@@ -44,7 +44,34 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=8, help="patches in the bounded CPU-baseline sample (0 = skip)")
     ap.add_argument("--eager-steps", type=int, default=10, help="timed steps of the torch-eager CUDA arm at N=1 (0 = skip)")
     ap.add_argument("--ops-out", default="", help="write the per-kernel timing breakdown (JSON) here")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0): infer = "
+                         "logits.npy (fp32 [n, classes, S, S]) and labels.npy (argmax as fp32 [n, S, S]) of n <= batch "
+                         "patches picked by a fixed seed, as many as fit in 63 MiB; train = loss.npy (fp64 [1])")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm only")
+    return a
+
+
+DUMP_BYTES = 63 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
+def sample_patches(logits, labels):
+    """logits [B, C, S, S] fp32 and labels [B, S, S] uint8 (device) -> the same fp32 rows of both for a seeded subset of
+    the batch that fits in DUMP_BYTES, as host arrays."""
+    import numpy as np
+    B, C, S, _ = logits.shape
+    n = min(B, DUMP_BYTES // ((C + 1) * S * S * 4))
+    idx = np.sort(np.random.default_rng(0).choice(B, n, replace=False)).tolist()
+    return {"logits": logits[idx].float().cpu().numpy(), "labels": labels[idx].float().cpu().numpy()}
 
 
 def peaks():
@@ -313,6 +340,9 @@ def run_train(a):
                           "note": "fp32 FMA peak of a B200 is ~72 TF/s (148 SMs x 128 lanes x 2 x 1.9 GHz); --train-gemm fp32 runs the "
                                   "trainable part on plain fp32 SIMT kernels (the gradient-parity tier)"}),
             "peak_mem_gb": torch.cuda.max_memory_allocated() / 2 ** 30}))
+        if a.dump_outputs:
+            import numpy as np
+            dump_outputs(a.dump_outputs, {"loss": np.array([float(loss)], dtype=np.float64)})
     if world > 1:
         dist.destroy_process_group()
 
@@ -449,10 +479,10 @@ def main():
     gat = AsyncGatherer(B * world, dev, torch.float16) if world > 1 else None
 
     def step(i):
-        logits, _ = eng.forward(xs[i % 3], use_graph=use_graph)
+        logits, labels = eng.forward(xs[i % 3], use_graph=use_graph)
         if gat is not None:
             gat.submit(logits)
-        return logits
+        return logits, labels
 
     with torch.no_grad(), ClockSampler(local) as clk:
         for i in range(W):
@@ -465,12 +495,14 @@ def main():
         t_region0 = time.perf_counter()
         e0.record()
         for i in range(K):
-            step(i)
+            last = step(i)
         if gat is not None:
             gat.wait_all()
         e1.record()
         torch.cuda.synchronize()
         t_region1 = time.perf_counter()
+        # the engine's output buffers are overwritten by the passes below: copy the sample out now
+        dumped = sample_patches(*last) if a.dump_outputs and rank == 0 else None
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
@@ -596,6 +628,8 @@ def main():
             "breakdown_ms": {k: round(v, 3) for k, v in list(breakdown.items())[:14]},
         }
         print(json.dumps(out))
+        if dumped is not None:
+            dump_outputs(a.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 

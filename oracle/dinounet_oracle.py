@@ -5,10 +5,11 @@ written against a flat state dict that uses the reference's own parameter names.
 the checker for the hand-written sm_100a kernels; only `tests/`, `__graft_entry__.smoke()`
 and `bench.py`'s cpu_baseline / `--impl reference` legs may import it.
 
-Parity pin: `tests/test_oracle_vs_reference.py` (runs where /root/reference exists) asserts
-this restatement is bit-identical (fp32, CPU) to the REAL reference forward imported through
-`oracle/ref_loader.py`, and `tests/golden/*.npz` (made by `oracle/make_golden.py` from the
-real reference) pins it on the GPU box where the reference is absent.
+Parity pin: on one host the restatement is bit-identical (fp32, CPU) to the REAL reference
+forward imported through `oracle/ref_loader.py`; `tests/test_oracle_vs_reference.py` and
+`tests/test_oracle_golden.py` hold it to the reference's outputs stored in `tests/golden/*.npz`
+(made by `oracle/make_golden.py` and `oracle/make_golden_reference_pins.py`) within fp32
+reduction-order noise.
 
 Reference locations followed (all relative to /root/reference):
   DinoUNet.forward                      dinounet_training.py:786-804

@@ -1,8 +1,9 @@
-"""TEST INFRASTRUCTURE ONLY — imports the REAL reference (`/root/reference`) on CPU.
+"""TEST INFRASTRUCTURE ONLY — imports the REAL reference (the original DinoUNet sources, at
+$DINOUNET_REFERENCE_ROOT) on CPU.
 
-Only usable in the build container (the GPU box has no /root/reference).  Used by
-`oracle/make_golden.py` and `tests/test_oracle_vs_reference.py` to pin the oracle
-restatement (`oracle/dinounet_oracle.py`) against the reference's own forward.
+Used by the golden generators (`oracle/make_golden.py`, `oracle/make_golden_reference_pins.py`) to pin the oracle
+restatement (`oracle/dinounet_oracle.py`) against the reference's own forward; the tests compare with what those
+generators stored under tests/golden/ and never need the reference itself.
 
 Shims (SURVEY.md §8c):
   1. `dinounet/__init__.py` pulls `api.py` -> batchgenerators (absent): pre-seed

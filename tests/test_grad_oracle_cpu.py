@@ -1,16 +1,15 @@
 """Gradient oracle (oracle/grad_oracle.py = autograd through the oracle forward + loss oracle), the round-2 backward
-target: pinned against autograd through the REAL reference module + REAL reference loss (build container only), and
-against committed golden gradient norms / samples (any container)."""
+target: pinned against autograd through the REAL reference module + REAL reference loss (stored in
+tests/golden/ref_pins_grads.npz), and against committed golden gradient norms / samples of the oracle itself."""
 import glob
 import os
 
 import numpy as np
-import pytest
 import torch
 
 from oracle import dinounet_oracle as O
 from oracle import grad_oracle as G
-from oracle.ref_loader import reference_available
+from oracle.make_golden_reference_pins import GRAD_CASE, strided_sample
 
 
 def _case(model, B, S, ncls, seed):
@@ -32,50 +31,46 @@ def test_grad_oracle_matches_golden():
         names = [str(n) for n in g["names"]]
         assert names == sorted(grads)
         norms = np.array([grads[k].double().norm().item() for k in names])
-        assert np.allclose(norms, g["norms"], rtol=1e-4, atol=1e-9)
+        # the conv biases ahead of an InstanceNorm have an exactly zero true gradient: their stored norms (below 1e-6 of
+        # the largest) are fp32 rounding noise that differs from host to host, so those only have to stay that small
+        floor = 1e-6 * g["norms"].max()
+        zero = g["norms"] < floor
+        assert (norms[zero] < floor).all(), [n for n, z, v in zip(names, zero, norms) if z and v >= floor]
+        assert np.allclose(norms[~zero], g["norms"][~zero], rtol=1e-4, atol=1e-9), \
+            [(n, v, w) for n, v, w in zip(names, norms, g["norms"]) if w >= floor and not np.isclose(v, w, rtol=1e-4, atol=1e-9)]
         for i, k in enumerate(names):
             fl = grads[k].reshape(-1)
             samp = fl[:: max(1, fl.numel() // 16)][:16].numpy()
             assert np.allclose(samp, g[f"s{i}"], rtol=1e-3, atol=1e-7), k
 
 
-@pytest.mark.skipif(not reference_available(), reason="needs /root/reference (build container only)")
 def test_grad_oracle_equals_reference_autograd():
-    from oracle.ref_loader import build_reference_model, load_reference_module
-    from oracle import loss_oracle as LO
-    import sys
-    model, ncls = "dinounet_s", 2
-    sd, x, target = _case(model, 1, 128, ncls, 3)
-    net = build_reference_model(model, ncls, sd)          # eval mode: BN running stats, DropPath off
-    load_reference_module()
-    msda_mod = sys.modules["dinounet.dinov3.eval.segmentation.models.utils.ms_deform_attn"]
-
-    class _Differentiable:                                 # the extension-backed backward cannot run on CPU (see module doc)
-        @staticmethod
-        def apply(value, shapes, lsi, loc, aw, step):
-            return msda_mod.ms_deform_attn_core_pytorch(value, shapes, loc, aw)
-
-    orig = msda_mod.MSDeformAttnFunction
-    msda_mod.MSDeformAttnFunction = _Differentiable
-    try:
-        DC_and_CE_loss, MemDice, _ = LO.load_reference_loss()
-        crit = DC_and_CE_loss({"batch_dice": True, "smooth": 1e-5, "do_bg": False, "ddp": False}, {}, weight_ce=1,
-                              weight_dice=1, ignore_label=None, dice_class=MemDice)
-        loss_ref = crit(net(x), target)
-        loss_ref.backward()
-    finally:
-        msda_mod.MSDeformAttnFunction = orig
+    """Against autograd through the reference module + reference loss (MSDA core swapped for its differentiable
+    pure-PyTorch twin, the extension's backward being CUDA-only), stored by oracle/make_golden_reference_pins.py: the loss,
+    the trainable-parameter set, and per tensor the absmax, the L2 norm and a strided sample of the gradient, each within
+    1e-4 of the tensor's scale.  The conv biases ahead of an InstanceNorm have an exactly zero true gradient; what
+    autograd leaves there (below 1e-6 of the largest gradient) is fp32 rounding noise that moves with the host's thread
+    count, so for those tensors the oracle's gradient must be as small, not equal."""
+    pins = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref_pins_grads.npz"))
+    model, B, S, ncls, seed = GRAD_CASE
+    sd, x, target = _case(model, B, S, ncls, seed)
     loss, grads = G.loss_and_grads(sd, model, x, target)
-    assert abs(loss.item() - loss_ref.item()) < 1e-6
-    ref = {n: p.grad for n, p in net.named_parameters() if p.requires_grad}
+    assert abs(loss.item() - float(pins["loss"])) < 1e-6
     # the reference's named_parameters() lists each shared Parameter once; every trainable oracle key must be among them
-    assert set(ref) == set(grads), (sorted(set(ref) ^ set(grads))[:10])
+    names = {str(n) for n in pins["names"]}
+    assert names == set(grads), (sorted(names ^ set(grads))[:10])
+    for k in pins["none"]:
+        assert float(grads[str(k)].abs().max()) == 0.0, k
+    floor = 1e-6 * float(pins["absmax"].max())
     worst = 0.0
-    for k, gr in ref.items():
-        go = grads[k]
-        if gr is None:
-            assert float(go.abs().max()) == 0.0, k
+    for i, k in enumerate(str(n) for n in pins["live"]):
+        go, amax, norm = grads[k], float(pins["absmax"][i]), float(pins["norm"][i])
+        if amax <= floor:
+            assert float(go.abs().max()) <= floor, k
             continue
-        denom = float(gr.abs().max()) + 1e-12
-        worst = max(worst, float((go - gr).abs().max()) / denom)
+        samp = strided_sample(go).numpy()
+        n = int(pins["n_samples"][i])
+        assert samp.size == n, k
+        worst = max(worst, float(np.abs(samp - pins["samples"][i, :n]).max()) / amax,
+                    abs(float(go.abs().max()) - amax) / amax, abs(go.double().norm().item() - norm) / norm)
     assert worst < 1e-4, worst

@@ -1,5 +1,5 @@
 """Sliding-window predictor, CPU side: the oracle restatement against the golden vectors produced by the REAL reference
-(`oracle/make_golden_sliding_window.py`), against the reference itself when it is present, and the product's host-side
+(`oracle/make_golden_sliding_window.py`, `oracle/make_golden_reference_pins.py`), and the product's host-side
 functions (steps, gaussian, padding, slicers, mirror order) against both."""
 import json
 import os
@@ -10,7 +10,7 @@ import pytest
 import torch
 
 from oracle import sliding_window_oracle as SWO
-from oracle.ref_loader import reference_available
+from oracle.make_golden_reference_pins import SW_CASES
 from dinounet_b200 import sliding_window as SW
 
 KAT = np.load(os.path.join(os.path.dirname(__file__), "golden", "sliding_window_kat.npz"))
@@ -64,14 +64,15 @@ def test_oracle_loop_matches_reference_golden_bitwise(case):
     assert y.dtype == torch.half and np.array_equal(y.numpy(), KAT[f"loop_{case}"])
 
 
-@pytest.mark.skipif(not reference_available(), reason="needs /root/reference (build container only)")
 def test_oracle_loop_matches_live_reference_predictor():
-    from oracle.make_golden_sliding_window import reference_loop
-    for seed, (shape, patch, step, ug, ma) in enumerate([((3, 2, 70, 45), (32, 32), 0.5, True, (0, 1)),
-                                                         ((1, 1, 100, 100), (64, 64), 0.3, True, (0,))]):
-        x, want = reference_loop(shape, patch, step, ug, ma, heads=3, seed=seed + 5)
-        got = SWO.predict_sliding_window_return_logits(toy_network(shape[0], 3, seed + 5), x, patch, 3, step, ug, ma)
-        assert torch.equal(got, want)
+    """nnUNetPredictor.predict_sliding_window_return_logits around a 3-head toy network, as run by
+    oracle/make_golden_reference_pins.py (input seeded like reference_loop's: seed + 1)."""
+    pins = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref_pins_sliding_window.npz"))
+    for k, (shape, patch, step, ug, ma) in enumerate(SW_CASES):
+        seed = k + 5
+        x = torch.randn(*shape, generator=torch.Generator().manual_seed(seed + 1))
+        got = SWO.predict_sliding_window_return_logits(toy_network(shape[0], 3, seed), x, patch, 3, step, ug, ma)
+        assert got.dtype == torch.half and np.array_equal(got.numpy(), pins[f"loop_{k}"])
 
 
 def test_product_padding_slicers_and_mirror_order():
